@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200 differentiable-A* engine.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload = BASELINE.json configs[1]: NeuralAstar inference (CNN encoder + differentiable A*),
@@ -14,6 +14,8 @@ per step in which the search kernel of batch k overlaps the encoder convolutions
 resident inputs (rotated through a ring larger than L2); `e2e` = the same loop with every step's inputs copied from
 pinned host memory and its results copied back (copies inside the graph).  Both are timed with CUDA events around
 the WHOLE K-step loop (pipeline fill and drain included), barrier + synchronize on both sides, max over ranks.
+Step k reads the 100 maps rolled by k % 112 positions, so the inputs of every step depend on k alone; `--dump-outputs DIR`
+saves what the last step returned (histories, paths) for output-for-output comparison of two builds.
 
 Prints ONE JSON line (rank 0) with the contract keys plus `roofline`, `cpu_baseline`, `e2e`, `clocks`,
 `gpu_launches`, and `configs` (BASELINE.json configs[2..4]: training step, WarCraft-shaped 12x12, 256x256).
@@ -82,6 +84,14 @@ def load_planner(device):
     msg = planner.load_state_dict({k: torch.from_numpy(state[k]) for k in state.files})
     assert not msg.missing_keys and not msg.unexpected_keys, msg
     return planner.to(device).eval()
+
+
+def dump_outputs(dirname, arrays):
+    """Write each array as <dirname>/<name>.npy (float32), so that two builds run with the same arguments can be
+    compared output for output."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -678,6 +688,9 @@ def bench_ours(args):
             return loop_dev(K, step_evs)
 
         total_ms, out = timer.loop(body)
+        # the last step's results live in graph-owned buffers that later replays overwrite: copy them now
+        dumped = ({"histories": out.histories.cpu().numpy(), "paths": out.paths.to(torch.float32).cpu().numpy()}
+                  if args.dump_outputs else None)
         launches = pipe_dev.native_launches - l0
         step_ms = [step_evs[i].elapsed_time(step_evs[i + 1]) for i in range(K)]
         e2e_ms, _ = timer.loop(lambda: loop_host(K))
@@ -790,6 +803,8 @@ def bench_ours(args):
             line["configs"] = configs
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = run_cpu_baseline()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if dist is not None:
         dist.barrier()
@@ -807,7 +822,14 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the configs block (training / WarCraft / 256x256)")
     ap.add_argument("--port", action="store_true", help="--impl reference: use the C restatement even if the reference is staged")
     ap.add_argument("--budget", type=float, default=150.0, help="--impl reference: seconds for warm-up + timed steps")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the histories and paths of the last timed step as DIR/histories.npy and DIR/paths.npy "
+                         "(float32, [100,1,32,32] each; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         bench_reference(args)
     else:
