@@ -6,13 +6,13 @@
 
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 #include "../../include/nastar_b200.h"
 #include "nastar_bin16.cuh"
 #include "nastar_generic.cuh"
 #include "nastar_glue.cuh"
-#include "nastar_warp32.cuh"
-#include "nastar_warp64.cuh"
+#include "nastar_warp.cuh"
 
 namespace {
 std::atomic<uint64_t> g_launches{0};
@@ -31,15 +31,15 @@ int num_sms() {
     return n;
 }
 
-// one-time fill of the 32x32 heuristic table on the current device (stream-ordered before first use)
-cudaError_t ensure_heur32(cudaStream_t stream) {
+// one-time fill of the warp engines' heuristic table on the current device (stream-ordered before first use)
+cudaError_t ensure_heur(cudaStream_t stream) {
     static std::atomic<uint64_t> done_mask{0};
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
     const uint64_t bit = uint64_t(1) << (dev & 63);
     if (done_mask.load(std::memory_order_acquire) & bit) return cudaSuccess;
-    nastar::heur32_init_kernel<<<4, 256, 0, stream>>>();
+    nastar::heur_init_kernel<<<nastar::kHeurCells / 256, 256, 0, stream>>>();
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     // later launches on OTHER streams must also see the table: finish the fill before publishing
@@ -50,20 +50,45 @@ cudaError_t ensure_heur32(cudaStream_t stream) {
     return cudaSuccess;
 }
 
-cudaError_t ensure_heur64(cudaStream_t stream) {
-    static std::atomic<uint64_t> done_mask{0};
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
+// Calls f with each runtime flag as a std::integral_constant<bool>, so that f can pick the kernel template
+// instantiation: with_flags(f, x, y) calls f(bool_constant<x>, bool_constant<y>).
+template <typename F>
+auto with_flags(F&& f) {
+    return f();
+}
+template <typename F, typename... Flags>
+auto with_flags(F&& f, bool first, Flags... rest) {
+    if (first) return with_flags([&](auto... c) { return f(std::true_type{}, c...); }, rest...);
+    return with_flags([&](auto... c) { return f(std::false_type{}, c...); }, rest...);
+}
+
+// the kernels' arguments for a backward call; the loop bound comes from *T_batch on the device (f.T = 0)
+nastar::SearchArgs backward_args(const nastar_bwd_params* p) {
+    nastar::SearchArgs a{};
+    a.f.cost = p->cost;   a.f.cost_stride = p->cost_stride;
+    a.f.start = p->start; a.f.start_stride = p->start_stride;
+    a.f.goal = p->goal;   a.f.goal_stride = p->goal_stride;
+    a.f.obst = p->obst;   a.f.obst_stride = p->obst_stride;
+    a.f.B = p->B; a.f.H = p->H; a.f.W = p->W;
+    a.f.g_ratio = p->g_ratio;
+    a.f.one_minus_g_ratio = p->one_minus_g_ratio;
+    a.f.workspace = p->workspace;
+    a.f.workspace_bytes = p->workspace_bytes;
+    a.sqrt_w = p->sqrt_w;
+    a.T_batch = p->T_batch;
+    a.t_solve_in = p->t_solve;
+    a.grad_hist = p->grad_histories;
+    a.grad_stride = p->grad_stride;
+    a.grad_cost = p->grad_cost;
+    return a;
+}
+
+// Launches kernel with `smem` bytes of dynamic shared memory (opting in above the 48 KB default).
+template <typename Kernel>
+cudaError_t launch_dyn(Kernel kernel, int grid, size_t smem, cudaStream_t stream, const nastar::SearchArgs& a) {
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return e;
-    const uint64_t bit = uint64_t(1) << (dev & 63);
-    if (done_mask.load(std::memory_order_acquire) & bit) return cudaSuccess;
-    nastar::heur64_init_kernel<<<16, 256, 0, stream>>>();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-    e = cudaStreamSynchronize(stream);
-    if (e != cudaSuccess) return e;
-    done_mask.fetch_or(bit, std::memory_order_release);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
+    kernel<<<grid, 32, smem, stream>>>(a);
     return cudaSuccess;
 }
 
@@ -205,42 +230,25 @@ int nastar_b200_forward(const nastar_fwd_params* p, void* stream_v) {
         cudaError_t e = cudaMemsetAsync(p->trace, 0xFF, size_t(nmaps) * size_t(p->T) * sizeof(int32_t), stream);
         if (e != cudaSuccess) return cuda_fail(e);
     }
-    if (engine == 1) {
-        cudaError_t he = ensure_heur32(stream);
-        if (he != cudaSuccess) return cuda_fail(he);
-        nastar::W32Args a{};
-        a.f = *p;
-        const bool noexit = (p->flags & NASTAR_FWD_NO_EARLY_EXIT) != 0;
-        const bool fused = (p->cost_kind != NASTAR_COST_PLANE);
-        auto go = [&](auto kernel) { kernel<<<nmaps, 32, 0, stream>>>(a); };
-        if (fused) {
-            if (p->trace) { if (noexit) go(nastar::astar_warp32_kernel<true, false, true, true>); else go(nastar::astar_warp32_kernel<true, false, false, true>); }
-            else          { if (noexit) go(nastar::astar_warp32_kernel<false, false, true, true>); else go(nastar::astar_warp32_kernel<false, false, false, true>); }
-        } else {
-            if (p->trace) { if (noexit) go(nastar::astar_warp32_kernel<true, false, true>); else go(nastar::astar_warp32_kernel<true, false, false>); }
-            else          { if (noexit) go(nastar::astar_warp32_kernel<false, false, true>); else go(nastar::astar_warp32_kernel<false, false, false>); }
-        }
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-    } else if (engine == 4) {
-        cudaError_t he = ensure_heur64(stream);
-        if (he != cudaSuccess) return cuda_fail(he);
-        const bool noexit = (p->flags & NASTAR_FWD_NO_EARLY_EXIT) != 0;
-        const size_t smem = sizeof(nastar::W64Smem);
-        nastar::W64Args wa{};
-        wa.f = *p;
-        auto launch = [&](auto kernel) -> cudaError_t {
-            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-            if (e != cudaSuccess) return e;
-            kernel<<<p->B, 32, smem, stream>>>(wa);
-            return cudaSuccess;
-        };
-        cudaError_t e;
-        if (p->cost_kind != NASTAR_COST_PLANE) {
-            if (p->trace) e = noexit ? launch(nastar::astar_warp64_kernel<true, true, false, true>) : launch(nastar::astar_warp64_kernel<true, false, false, true>);
-            else e = noexit ? launch(nastar::astar_warp64_kernel<false, true, false, true>) : launch(nastar::astar_warp64_kernel<false, false, false, true>);
-        } else if (p->trace) e = noexit ? launch(nastar::astar_warp64_kernel<true, true>) : launch(nastar::astar_warp64_kernel<true, false>);
-        else e = noexit ? launch(nastar::astar_warp64_kernel<false, true>) : launch(nastar::astar_warp64_kernel<false, false>);
+    const bool trace = (p->trace != nullptr);
+    const bool noexit = (p->flags & NASTAR_FWD_NO_EARLY_EXIT) != 0;
+    const bool fused = (p->cost_kind != NASTAR_COST_PLANE);
+    if (engine == 1 || engine == 4) {
+        cudaError_t e = ensure_heur(stream);
         if (e != cudaSuccess) return cuda_fail(e);
+        nastar::SearchArgs a{};
+        a.f = *p;
+        if (engine == 1) {
+            with_flags([&](auto kTrace, auto kNoExit, auto kFused) {
+                nastar::astar_warp32_kernel<kTrace, false, kNoExit, kFused><<<nmaps, 32, 0, stream>>>(a);
+            }, trace, noexit, fused);
+        } else {
+            e = with_flags([&](auto kTrace, auto kNoExit, auto kFused) {
+                return launch_dyn(nastar::astar_warp64_kernel<kTrace, false, kNoExit, kFused>, p->B,
+                                  sizeof(nastar::WarpSmem<64>), stream, a);
+            }, trace, noexit, fused);
+            if (e != cudaSuccess) return cuda_fail(e);
+        }
         g_launches.fetch_add(1, std::memory_order_relaxed);
     } else {
         const nastar::GenericLayout L(p->H, p->W);
@@ -252,7 +260,7 @@ int nastar_b200_forward(const nastar_fwd_params* p, void* stream_v) {
             grid = generic_slots(p->B);
             if (!p->workspace || p->workspace_bytes < slots_bytes) return NASTAR_EWORKSPACE;
         }
-        nastar::GenArgs ga{};
+        nastar::SearchArgs ga{};
         ga.f = *p;
         // engine 5 first when the cost plane IS the binary obstacle plane (VanillaAstar / Config 5): whole map on
         // chip, one CTA per SM pulling maps from a queue; maps it flags are re-run below by the generic engine
@@ -286,21 +294,9 @@ int nastar_b200_forward(const nastar_fwd_params* p, void* stream_v) {
             ga.f.workspace = ws + aux;
             ga.f.workspace_bytes = p->workspace_bytes - aux;
         }
-        auto launch = [&](auto kernel) -> cudaError_t {
-            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-            if (e != cudaSuccess) return e;
-            kernel<<<grid, 32, smem, stream>>>(ga);
-            return cudaSuccess;
-        };
-        const bool noexit = (p->flags & NASTAR_FWD_NO_EARLY_EXIT) != 0;
-        cudaError_t e;
-        if (noexit) {
-            if (global) e = p->trace ? launch(nastar::astar_generic_kernel<true, true, false, true>) : launch(nastar::astar_generic_kernel<true, false, false, true>);
-            else e = p->trace ? launch(nastar::astar_generic_kernel<false, true, false, true>) : launch(nastar::astar_generic_kernel<false, false, false, true>);
-        } else {
-            if (global) e = p->trace ? launch(nastar::astar_generic_kernel<true, true, false>) : launch(nastar::astar_generic_kernel<true, false, false>);
-            else e = p->trace ? launch(nastar::astar_generic_kernel<false, true, false>) : launch(nastar::astar_generic_kernel<false, false, false>);
-        }
+        const cudaError_t e = with_flags([&](auto kGlobal, auto kTrace, auto kNoExit) {
+            return launch_dyn(nastar::astar_generic_kernel<kGlobal, kTrace, false, kNoExit>, grid, smem, stream, ga);
+        }, global, trace, noexit);
         if (e != cudaSuccess) return cuda_fail(e);
         g_launches.fetch_add(1, std::memory_order_relaxed);
     }
@@ -315,103 +311,30 @@ int nastar_b200_backward(const nastar_bwd_params* p, void* stream_v) {
         return NASTAR_EINVAL;
     if (p->B <= 0 || p->H <= 0 || p->W <= 0) return NASTAR_EINVAL;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
-    int engine = nastar_b200_engine_for(p->H, p->W);
-    if (engine == 4) {
-        // warp-resident 64-wide engine: event-based closed form next to the forward state in shared memory
-        cudaError_t he = ensure_heur64(stream);
-        if (he != cudaSuccess) return cuda_fail(he);
-        nastar::W64Args wa{};
-        wa.f.cost = p->cost;   wa.f.cost_stride = p->cost_stride;
-        wa.f.start = p->start; wa.f.start_stride = p->start_stride;
-        wa.f.goal = p->goal;   wa.f.goal_stride = p->goal_stride;
-        wa.f.obst = p->obst;   wa.f.obst_stride = p->obst_stride;
-        wa.f.B = p->B; wa.f.H = p->H; wa.f.W = p->W;
-        wa.f.g_ratio = p->g_ratio;
-        wa.f.one_minus_g_ratio = p->one_minus_g_ratio;
-        wa.f.T = 0;   // the loop bound comes from *T_batch on the device
-        wa.sqrt_w = p->sqrt_w;
-        wa.T_batch = p->T_batch;
-        wa.t_solve_in = p->t_solve;
-        wa.grad_hist = p->grad_histories;
-        wa.grad_stride = p->grad_stride;
-        wa.grad_cost = p->grad_cost;
-        const size_t smem = sizeof(nastar::W64Smem) + sizeof(nastar::W64Bwd);
-        cudaError_t e = cudaFuncSetAttribute(nastar::astar_warp64_kernel<false, false, true>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-        if (e != cudaSuccess) return cuda_fail(e);
-        nastar::astar_warp64_kernel<false, false, true><<<p->B, 32, smem, stream>>>(wa);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        e = cudaGetLastError();
-        if (e != cudaSuccess) return cuda_fail(e);
-        return NASTAR_OK;
-    }
-    if (engine != 1) engine = generic_engine_for(p->H, p->W);
+    const int engine = nastar_b200_engine_for(p->H, p->W);
     if (engine == 0) return NASTAR_EUNSUPPORTED;
-    if (engine >= 2) {
+    const nastar::SearchArgs a = backward_args(p);
+    cudaError_t e;
+    if (engine == 1 || engine == 4) {
+        e = ensure_heur(stream);
+        if (e != cudaSuccess) return cuda_fail(e);
+        // the event-based closed form keeps its per-cell interval state in dynamic shared memory (WarpBwd): 32 KB
+        // next to the warp32 engine's 17.4 KB of static planes, 128 KB behind the warp64 engine's planes
+        if (engine == 1) e = launch_dyn(nastar::astar_warp32_kernel<false, true>, p->B, sizeof(nastar::WarpBwd<32>), stream, a);
+        else e = launch_dyn(nastar::astar_warp64_kernel<false, true>, p->B, sizeof(nastar::WarpSmem<64>) + sizeof(nastar::WarpBwd<64>), stream, a);
+    } else {
         const nastar::GenericLayout L(p->H, p->W);
         const bool global = (engine == 3);
         const int grid = generic_slots(p->B);
         if (!p->workspace || p->workspace_bytes < size_t(grid) * L.slot_total(global, true)) return NASTAR_EWORKSPACE;
-        nastar::GenArgs ga{};
-        ga.f.cost = p->cost;   ga.f.cost_stride = p->cost_stride;
-        ga.f.start = p->start; ga.f.start_stride = p->start_stride;
-        ga.f.goal = p->goal;   ga.f.goal_stride = p->goal_stride;
-        ga.f.obst = p->obst;   ga.f.obst_stride = p->obst_stride;
-        ga.f.B = p->B; ga.f.H = p->H; ga.f.W = p->W;
-        ga.f.g_ratio = p->g_ratio;
-        ga.f.one_minus_g_ratio = p->one_minus_g_ratio;
-        ga.f.workspace = p->workspace;
-        ga.f.workspace_bytes = p->workspace_bytes;
-        ga.sqrt_w = p->sqrt_w;
-        ga.T_batch = p->T_batch;
-        ga.t_solve_in = p->t_solve;
-        ga.grad_hist = p->grad_histories;
-        ga.grad_stride = p->grad_stride;
-        ga.grad_cost = p->grad_cost;
         const size_t smem = L.smem_common() + (global ? 0 : L.smem_planes());
-        cudaError_t e;
-        if (global) {
-            e = cudaFuncSetAttribute(nastar::astar_generic_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-            if (e == cudaSuccess) nastar::astar_generic_kernel<true, false, true><<<grid, 32, smem, stream>>>(ga);
-        } else {
-            e = cudaFuncSetAttribute(nastar::astar_generic_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-            if (e == cudaSuccess) nastar::astar_generic_kernel<false, false, true><<<grid, 32, smem, stream>>>(ga);
-        }
-        if (e != cudaSuccess) return cuda_fail(e);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        e = cudaGetLastError();
-        if (e != cudaSuccess) return cuda_fail(e);
-        return NASTAR_OK;
+        e = with_flags([&](auto kGlobal) {
+            return launch_dyn(nastar::astar_generic_kernel<kGlobal, false, true>, grid, smem, stream, a);
+        }, global);
     }
-    {
-        cudaError_t he = ensure_heur32(stream);
-        if (he != cudaSuccess) return cuda_fail(he);
-    }
-    nastar::W32Args a{};
-    a.f.cost = p->cost;   a.f.cost_stride = p->cost_stride;
-    a.f.start = p->start; a.f.start_stride = p->start_stride;
-    a.f.goal = p->goal;   a.f.goal_stride = p->goal_stride;
-    a.f.obst = p->obst;   a.f.obst_stride = p->obst_stride;
-    a.f.B = p->B; a.f.H = p->H; a.f.W = p->W;
-    a.f.g_ratio = p->g_ratio;
-    a.f.one_minus_g_ratio = p->one_minus_g_ratio;
-    a.f.T = 0;  // the loop bound comes from *T_batch on the device
-    a.sqrt_w = p->sqrt_w;
-    a.T_batch = p->T_batch;
-    a.t_solve_in = p->t_solve;
-    a.grad_hist = p->grad_histories;
-    a.grad_stride = p->grad_stride;
-    a.grad_cost = p->grad_cost;
-    // dynamic shared memory = the per-cell interval state of the event-based closed form (W32Bwd, 32 KB); with the
-    // 17.4 KB of static planes that is above the 48 KB default, hence the opt-in
-    {
-        cudaError_t ea = cudaFuncSetAttribute(nastar::astar_warp32_kernel<false, true>,
-                                              cudaFuncAttributeMaxDynamicSharedMemorySize, int(sizeof(nastar::W32Bwd)));
-        if (ea != cudaSuccess) return cuda_fail(ea);
-    }
-    nastar::astar_warp32_kernel<false, true><<<p->B, 32, sizeof(nastar::W32Bwd), stream>>>(a);
+    if (e != cudaSuccess) return cuda_fail(e);
     g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t e = cudaGetLastError();
+    e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e);
     return NASTAR_OK;
 }

@@ -7,10 +7,27 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/nastar_b200.h"
+
 namespace nastar {
 
 constexpr unsigned kFull = 0xFFFFFFFFu;
 constexpr uint32_t kKeyInf = 0xFFFFFFFFu;  // "no open cell" sentinel, above every float key
+
+// Kernel arguments of every search engine: the forward parameters plus the extra fields of nastar_bwd_params.
+struct SearchArgs {
+    nastar_fwd_params f;
+    // backward only
+    float sqrt_w;
+    const int32_t* T_batch;     // device scalar: loop iterations the reference would execute
+    const int32_t* t_solve_in;  // forward's t_solve[] (goal clamp blocking, App. B)
+    const float* grad_hist;
+    int64_t grad_stride;
+    float* grad_cost;
+    // generic engine, forward only, nullable: per-map flags written by the bin16 engine (nastar_bin16.cuh); when
+    // given, only maps with redo[b] != 0 are processed (the others were already finished on-chip)
+    const int32_t* redo;
+};
 
 // Order-preserving map float -> uint32 (a < b  <=>  key(a) < key(b) for non-NaN a, b).
 __device__ __forceinline__ uint32_t fkey(float f) {
@@ -79,6 +96,46 @@ __device__ __forceinline__ void dd_add(double& hi, double& lo, double x) {
     lo = __dadd_rn(lo, -__dadd_rn(t, -s));
     hi = t;
 }
+
+// Per-cell state of the event-based backward (SURVEY App. B), in shared memory or in a workspace slot.
+// dL/dcost[p] = -(1-g_ratio)/sqrt(W) * sum_t y_t[p] * (Gh[p] - <Gh, y_t>) with y_t = v_t / S_t over the open set.
+// A cell's softmax weight v = exp(-f/sqrt(W)) only changes when it is opened, relaxed or closed, so its contribution
+// over an interval [t0, t1) of constant v is v * (Gh * (A(t1)-A(t0)) - (B(t1)-B(t0))) with the prefix sums
+// A(t) = sum_{tau<t} 1/S_tau and B(t) = sum_{tau<t} D_tau/S_tau^2, D_t = <Gh, v_t>.
+struct IntervalPlanes {
+    double* acc;  // closed intervals: sum of v * (Gh * dA - dB)
+    double* a0;   // A(t0), B(t0) of the cell's current open interval
+    double* b0;
+    float* v;     // softmax numerator of open cells, else 0
+
+    // The weight of cell i changes to v_new (0: the cell leaves the open set) from the next step on; A1, B1 are the
+    // prefix sums including the current step.  Returns the change of v.
+    __device__ __forceinline__ double event(int i, double gh, float v_new, double A1, double B1) const {
+        const float v_old = v[i];
+        if (v_old != 0.f) acc[i] += double(v_old) * (gh * (A1 - a0[i]) - (B1 - b0[i]));
+        v[i] = v_new;
+        a0[i] = A1;
+        b0[i] = B1;
+        return double(v_new) - double(v_old);
+    }
+    // The open cell i is closed (the generic engine's selection event): its last interval ends at A1, B1; A(t0) and
+    // B(t0) are left stale, a closed cell is never reopened.  Returns the change of v.
+    __device__ __forceinline__ double leave(int i, double gh, double A1, double B1) const {
+        const float v_old = v[i];
+        acc[i] += double(v_old) * (gh * (A1 - a0[i]) - (B1 - b0[i]));
+        v[i] = 0.f;
+        return -double(v_old);
+    }
+    // acc of cell i with its open interval (if any) closed at the end of the search, prefix sums A, B; gh_at() gives
+    // the cell's upstream gradient and is only evaluated for open cells
+    template <typename GhAt>
+    __device__ __forceinline__ double close(int i, double A, double B, GhAt gh_at) const {
+        double r = acc[i];
+        const float vi = v[i];
+        if (vi != 0.f) r += double(vi) * (gh_at() * (A - a0[i]) - (B - b0[i]));
+        return r;
+    }
+};
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));

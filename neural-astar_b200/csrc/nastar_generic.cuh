@@ -39,36 +39,13 @@ struct GenericLayout {
     }
 };
 
-// forward parameters + the extra fields of nastar_bwd_params (same idea as W32Args)
-struct GenArgs {
-    nastar_fwd_params f;
-    float sqrt_w;
-    const int32_t* T_batch;
-    const int32_t* t_solve_in;
-    const float* grad_hist;
-    int64_t grad_stride;
-    float* grad_cost;
-    // forward only, nullable: per-map flags written by the bin16 engine (nastar_bin16.cuh); when given, only
-    // maps with redo[b] != 0 are processed here (the others were already finished on-chip)
-    const int32_t* redo;
-};
-
-__device__ __forceinline__ float gen_warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
-    return v;
-}
-
 // kBwd = true replays the search for *T_batch steps and accumulates the closed-form gradient (SURVEY App. B)
-//   dL/dcost[p] = -(1-g_ratio)/sqrt(W) * sum_t y_t[p] * (Gh[p] - <Gh, y_t>),   y_t = v_t / S_t over the open set,
-// EVENT-BASED: v_t[p] = exp(-f_t[p]/sqrt(W)) only changes when p is opened, relaxed or closed, so a cell's
-// contribution over an interval [t0, t1) of constant v is v * (Gh[p] * (A(t1)-A(t0)) - (B(t1)-B(t0))) with the
-// prefix sums A(t) = sum_{tau<t} 1/S_tau, B(t) = sum_{tau<t} D_tau/S_tau^2, D_t = <Gh, v_t>.  S and D are
-// maintained incrementally in fp64 from the <= 9 events of a step — O(1) work per step instead of a dense
-// O(N/32) softmax pass (round 1).  Per-cell state (v, A(t0), B(t0), acc) lives in the per-CTA workspace slot.
+// EVENT-BASED (IntervalPlanes, nastar_common.cuh): S and D are maintained incrementally in fp64 from the <= 9 events
+// of a step — O(1) work per step instead of a dense O(N/32) softmax pass (round 1).  Per-cell state (v, A(t0), B(t0),
+// acc) lives in the per-CTA workspace slot.
 // kNoExit (forward only): NASTAR_FWD_NO_EARLY_EXIT — keep stepping after the solve step, exactly T steps.
 template <bool kGlobal, bool kTrace, bool kBwd, bool kNoExit = false>
-__global__ void __launch_bounds__(32) astar_generic_kernel(const GenArgs a) {
+__global__ void __launch_bounds__(32) astar_generic_kernel(const SearchArgs a) {
     constexpr bool kContinue = kBwd || kNoExit;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const nastar_fwd_params& p = a.f;
@@ -94,17 +71,14 @@ __global__ void __launch_bounds__(32) astar_generic_kernel(const GenArgs a) {
         F = G + np;
         Par = reinterpret_cast<uint8_t*>(F + np);
     }
-    float* V = nullptr;     // backward: v = exp(-f/sqrt(W)) of open cells, else 0
-    double* ACC = nullptr;  // backward: sum over closed intervals of v * (Gh * dA - dB)
-    double* A0 = nullptr;   // backward: A(t0), B(t0) of the cell's current interval
-    double* B0 = nullptr;
+    IntervalPlanes iv{};    // backward only
     if (kBwd) {
         unsigned char* slot = static_cast<unsigned char*>(p.workspace) + size_t(blockIdx.x) * L.slot_total(kGlobal, true) +
                               (kGlobal ? L.slot_bytes() : 0);
-        ACC = reinterpret_cast<double*>(slot);
-        A0 = ACC + np;
-        B0 = A0 + np;
-        V = reinterpret_cast<float*>(B0 + np);
+        iv.acc = reinterpret_cast<double*>(slot);
+        iv.a0 = iv.acc + np;
+        iv.b0 = iv.a0 + np;
+        iv.v = reinterpret_cast<float*>(iv.b0 + np);
     }
     uint32_t* sPass = reinterpret_cast<uint32_t*>(sp); sp += size_t(L.nbits) * 4;
     uint32_t* sOpen = reinterpret_cast<uint32_t*>(sp); sp += size_t(L.nbits) * 4;
@@ -231,7 +205,7 @@ __global__ void __launch_bounds__(32) astar_generic_kernel(const GenArgs a) {
             ts_in = a.t_solve_in[b];
             blocked = (ts_in >= 0) && (ts_in < Tb - 1);   // goal clamp, differentiable_astar.py:222-223
             gG = a.grad_hist + int64_t(b) * a.grad_stride;
-            for (int i = lane; i < N; i += 32) { V[i] = 0.f; ACC[i] = 0.0; }
+            for (int i = lane; i < N; i += 32) { iv.v[i] = 0.f; iv.acc[i] = 0.0; }
             __syncwarp();
         }
         // backward running sums (replicated in every lane): S = sum of v over the open set, D = <Gh, v>,
@@ -244,14 +218,14 @@ __global__ void __launch_bounds__(32) astar_generic_kernel(const GenArgs a) {
             const float f0 = f_value(gr, omg, 0.f, h0);
             G[start_idx] = 0.f;
             F[start_idx] = f0;
-            if (kBwd) { V[start_idx] = expf(__fdiv_rn(-f0, a.sqrt_w)); A0[start_idx] = 0.0; B0[start_idx] = 0.0; }
+            if (kBwd) { iv.v[start_idx] = expf(__fdiv_rn(-f0, a.sqrt_w)); iv.a0[start_idx] = 0.0; iv.b0[start_idx] = 0.0; }
             sOpen[sy * Wd + (sx >> 5)] = 1u << (sx & 31);
             sRmKey[sy] = fkey(f0);
             sRmCol[sy] = sx;
         }
         __syncwarp();
         if (kBwd && start_idx >= 0) {
-            Ssum = double(V[start_idx]);
+            Ssum = double(iv.v[start_idx]);
             Dsum = double(gh_at(start_idx)) * Ssum;
         }
         uint32_t bk = kKeyInf;
@@ -333,25 +307,17 @@ __global__ void __launch_bounds__(32) astar_generic_kernel(const GenArgs a) {
                 atomicOr(&sOpen[y * Wd + (x >> 5)], 1u << (x & 31));
                 key = fkey(fn);
                 if (kBwd) {
-                    // event: the cell's softmax weight changes from v_old (0 if it was not open) to v_new after this step
-                    const float v_old = V[n], v_new = expf(__fdiv_rn(-fn, a.sqrt_w));
+                    const float v_new = expf(__fdiv_rn(-fn, a.sqrt_w));
                     const double gh = double(gh_at(n));
-                    if (v_old != 0.f) ACC[n] += double(v_old) * (gh * (A1 - A0[n]) - (B1 - B0[n]));
-                    V[n] = v_new;
-                    A0[n] = A1;
-                    B0[n] = B1;
-                    dS = double(v_new) - double(v_old);
+                    dS = iv.event(n, gh, v_new, A1, B1);
                     dD = gh * dS;
                 }
             }
             if (kBwd) {
                 if (lane == 9 && !solved) {
                     // event: the selected cell leaves the open set (the goal stays open, :224)
-                    const float v_old = V[ind];
                     const double gh = double(gh_at(ind));
-                    ACC[ind] += double(v_old) * (gh * (A1 - A0[ind]) - (B1 - B0[ind]));
-                    V[ind] = 0.f;
-                    dS = -double(v_old);
+                    dS = iv.leave(ind, gh, A1, B1);
                     dD = gh * dS;
                 }
 #pragma unroll
@@ -404,12 +370,7 @@ __global__ void __launch_bounds__(32) astar_generic_kernel(const GenArgs a) {
             // close the intervals of the cells still open at the end, then scale
             const float coef = -omg / a.sqrt_w;
             float* gOut = a.grad_cost + int64_t(b) * N;
-            for (int i = lane; i < N; i += 32) {
-                double acc = ACC[i];
-                const float v = V[i];
-                if (v != 0.f) acc += double(v) * (double(gh_at(i)) * (Acum - A0[i]) - (Bcum - B0[i]));
-                gOut[i] = float(double(coef) * acc);
-            }
+            for (int i = lane; i < N; i += 32) gOut[i] = float(double(coef) * iv.close(i, Acum, Bcum, [&] { return double(gh_at(i)); }));
             __syncwarp();
         }
         if (!kBwd) {
